@@ -7,6 +7,7 @@ A "step" = one pass of the hot path over that batch: layout pre-pass (NCHW -> ch
 texels) + ray generation + ImportanceRenderer.forward.  Synthetic data, random-init decoder.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]           our arm (CUDA, one rank per GPU)
+    python bench.py [...] --dump-outputs DIR                      also write the last timed step's outputs as DIR/*.npy
     python bench.py --impl reference [...]                        the reference's CPU algorithm (oracle port)
 
 Prints ONE JSON line (rank 0).  See DESIGN.md section "Measurement" for how every field is derived.
@@ -259,12 +260,14 @@ def run_ours(args):
     gather_buf = torch.empty((world * VIEWS, R * R, 32), device=dev) if gather_mode == 'nccl' else None
     peer = pviews.PeerGather((VIEWS, R * R, 32), torch.float32, dev, dst=0) if gather_mode == 'p2p' else None
     step_no = [0]
+    last = {}                                                                 # the most recent step's results, for --dump-outputs
 
     def step():
         c2w, K = labels_dev[:, :16].view(-1, 4, 4), labels_dev[:, 16:25].view(-1, 3, 3)
         ro, rd = sampler(c2w, K, R)
         renderer._planes.key = None                                           # distinct tri-planes every step: redo the layout pass
         rgb, depth, wsum, xyz = renderer(planes, decoder, ro, rd, opts)
+        last.update(ray_origins=ro, ray_directions=rd, rgb=rgb, depth=depth, weights_sum=wsum, xyz=xyz)
         if gather_mode == 'nccl':
             dist.all_gather_into_tensor(gather_buf, rgb)
         elif gather_mode == 'p2p':
@@ -295,6 +298,8 @@ def run_ours(args):
         barrier()
         ms = e0.elapsed_time(e1)
         launches = _lib.launch_count() - n0
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, last)
     with torch.no_grad():
         # ---- per-kernel device time for the roofline (separate short run with event brackets enabled)
         L.p3d_profile_enable(1)
@@ -544,6 +549,16 @@ def run_e2e(L, _lib, planes, decoder, labels, opts, mlp_mode, args, barrier):
     return {'ms': ms, 'steps': steps, 'h2d': h2d, 'd2h': d2h}
 
 
+def dump_outputs(out_dir, tensors):
+    """Write each tensor as out_dir/<name>.npy in float32, whole: the last timed step's rays and the four renderer outputs
+    come to 22.5 MB.  The inputs are seeded (tri-planes, decoder, cameras, and the per-call jitter seed drawn from the
+    torch CPU generator), so the same command line renders the same step on every build."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in tensors.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.detach().float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -556,7 +571,14 @@ def main():
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-variants', action='store_true', help='skip the 48+48 / bf16 / fp32_simt context measurements')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the last timed step\'s ray origins / directions and rgb / depth / '
+                         'weights_sum / xyz (rank 0\'s views) as DIR/<name>.npy, float32')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.impl == 'reference' and args.dump_outputs:
+        ap.error('--dump-outputs writes what the CUDA arm computed; it does not apply to --impl reference')
     if args.impl == 'reference':
         run_reference(args)
     else:

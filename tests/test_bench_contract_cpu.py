@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -29,6 +31,12 @@ def test_reference_arm_prints_the_contract_line():
     assert d['config'] == bench.workload_config(1, 'tc_3xbf16', 'fp32') and d['warmup'] == 1
     assert d['e2e'] == {'value': d['value'], 'unit': 'views/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}
     assert d['gpu_launches'] == 0
+
+
+@pytest.mark.parametrize('argv', [['--steps', '0'], ['--impl', 'reference', '--dump-outputs', 'out']])
+def test_bench_rejects_arguments_it_cannot_honour(argv, tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py')] + argv, capture_output=True, text=True, timeout=60, cwd=tmp_path)
+    assert r.returncode == 2 and 'error:' in r.stderr and not os.listdir(tmp_path)
 
 
 def test_gpu_arm_of_bench_does_not_touch_the_oracle():

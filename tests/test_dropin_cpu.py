@@ -1,14 +1,11 @@
-"""CPU: the drop-in mechanism.  With the reference tree present (build container only) the reference's own
-TriPlaneGenerator must pick up this package's renderer / ray sampler by import name, unchanged."""
+"""CPU: the drop-in mechanism.  The reference's own TriPlaneGenerator must pick up this package's renderer / ray sampler
+by import name, unchanged."""
 import os
 import subprocess
 import sys
 import textwrap
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = '/root/reference'
 
 
 def test_install_registers_modules():
@@ -26,42 +23,55 @@ def test_install_registers_modules():
     assert r.returncode == 0 and 'ok' in r.stdout, r.stderr[-2000:]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree only exists in the build container')
 def test_reference_generator_uses_dropin_modules():
+    """The reference's TriPlaneGenerator reaches the renderer and ray sampler by import name and ``paste_front`` by module
+    global.  tests/golden/dropin_reference.json records those names, the constructor and hook signatures and what a built
+    generator holds, from the unmodified reference (tests/golden/make_golden_dropin.py): after install() / install_paste()
+    every name resolves to this package, and this package's classes and hooks match what was recorded."""
     code = textwrap.dedent('''
-        import os, sys, types
-        os.environ['PROJECT_DN'] = %(ref)r
-        sys.path[:0] = [%(root)r, %(ref)r, %(ref)r + '/_train/eg3dc/src']
-        sys.modules['kornia'] = types.ModuleType('kornia')
+        import importlib, inspect, json, sys, types
+        sys.path.insert(0, %(root)r)
+        ref = json.load(open(%(golden)r))
         import panic3d_b200.dropin as d
-        d.install(ops=False)
-        import training.triplane as tp                       # the reference's own file
-        assert tp.__file__.startswith(%(ref)r)
+        served = d.install()
         import panic3d_b200.training.volumetric_rendering.renderer as ours_r
         import panic3d_b200.training.volumetric_rendering.ray_sampler as ours_s
-        assert tp.ImportanceRenderer is ours_r.ImportanceRenderer
-        assert tp.RaySampler is ours_s.RaySampler
-        rk = dict(superresolution_module='training.superresolution.SuperresolutionHybrid8XDC', sr_antialias=True,
-                  use_triplane=True, c_gen_conditioning_zero=True, decoder_lr_mul=1, box_warp=0.7)
-        G = tp.TriPlaneGenerator(z_dim=64, c_dim=25, w_dim=64, img_resolution=512, img_channels=3, rendering_kwargs=rk,
-                                 cond_mode='none', mapping_kwargs=dict(num_layers=1), channel_base=2048, channel_max=32,
-                                 sr_kwargs=dict(channel_base=2048, channel_max=32, fused_modconv_default='inference_only'))
-        assert type(G.renderer) is ours_r.ImportanceRenderer and G.renderer.use_triplane
-        assert type(G.ray_sampler) is ours_s.RaySampler
-        assert sum(p.numel() for p in G.renderer.parameters()) == 0
-        assert tuple(G.decoder.net[0].weight.shape) == (64, 32) and tuple(G.decoder.net[2].weight.shape) == (33, 64)
-        # SURVEY 8f-3: G.f resolves `paste_front` in its module's globals at call time (triplane.py:498-502), so rebinding the
-        # module attribute is the whole plug-in
-        import inspect
+        import panic3d_b200.training.triplane as ours_tp
         import panic3d_b200.paste as ours_p
+        ours = {'ImportanceRenderer': ours_r.ImportanceRenderer, 'RaySampler': ours_s.RaySampler}
+        for name, mod in ref['triplane_imports'].items():            # triplane.py: `from <mod> import <name>`
+            assert getattr(importlib.import_module(mod), name) is ours[name], (name, mod)
+        # every renderer module the reference loads is served, and every served module is one the reference loads
+        assert sorted(m for m in served if m.startswith('training.')) == \\
+            [m for m in ref['modules_loaded'] if m.startswith('training.volumetric_rendering.')], served
+        assert set(served) <= set(ref['modules_loaded']), served
+        params = lambda fn: [[p.name, p.kind.name, None if p.default is inspect.Parameter.empty else repr(p.default)]
+                             for p in inspect.signature(fn).parameters.values()]
+        assert params(ours_r.ImportanceRenderer.__init__)[1:] == ref['renderer_init']
+        assert params(ours_s.RaySampler.__init__)[1:] == ref['ray_sampler_init']
+        gen = ref['generator']                                       # built with rendering_kwargs use_triplane=True
+        renderer, sampler = ours_r.ImportanceRenderer(use_triplane=True), ours_s.RaySampler()
+        assert renderer.plane_axes.tolist() == gen['renderer_plane_axes']
+        assert sum(p.numel() for p in renderer.parameters()) == gen['renderer_parameters']
+        assert sum(p.numel() for p in sampler.parameters()) == gen['ray_sampler_parameters']
+        dec = ours_tp.OSGDecoder(32, {'decoder_lr_mul': 1, 'decoder_output_dim': 32})
+        assert {n: list(p.shape) for n, p in dec.named_parameters()} == gen['decoder_parameters']
+        assert all(hasattr(dec.net[i], a) for i in (0, 2) for a in gen['decoder_gains'])
+        # G.f resolves `paste_front` in its module's globals at call time, so rebinding the module attribute is the whole
+        # plug-in: a stand-in `training.triplane` whose f calls the recorded globals
+        tp = types.ModuleType('training.triplane')
+        for name in ref['hooks']:
+            setattr(tp, name, lambda *a, **k: 'reference')
+        exec('def f(*a):\\n    return [%%s]\\n' %% ', '.join(n + '(*a)' for n in ref['f_module_globals']), tp.__dict__)
+        sys.modules['training.triplane'] = tp
         ref_paste = tp.paste_front
-        assert 'paste = paste_front(self, x, ret, **x[' in inspect.getsource(tp.TriPlaneGenerator.f)
-        assert d.install_paste() == ['paste_front', 'get_front_occlusion', 'get_front_weights']     # finds training.triplane by name
+        assert d.install_paste() == list(ref['hooks'])               # finds training.triplane by name
         assert tp.paste_front is ours_p.paste_front and tp._p3d_reference_paste_front is ref_paste
-        assert tp.TriPlaneGenerator.f.__globals__['paste_front'] is ours_p.paste_front
-        assert list(inspect.signature(ours_p.paste_front).parameters)[:12] == list(inspect.signature(ref_paste).parameters)[:12]
+        assert tp.f.__globals__['paste_front'] is ours_p.paste_front and ref['f_module_globals'] == ['paste_front']
+        for name, want in ref['hooks'].items():
+            assert getattr(tp, name) is getattr(ours_p, name) and params(getattr(ours_p, name)) == want, name
         print('ok')
-    ''' % dict(root=ROOT, ref=REF))
+    ''' % dict(root=ROOT, golden=os.path.join(ROOT, 'tests', 'golden', 'dropin_reference.json')))
     r = subprocess.run([sys.executable, '-c', code], capture_output=True, text=True)
     assert r.returncode == 0 and 'ok' in r.stdout, (r.stdout[-1000:], r.stderr[-3000:])
 
