@@ -1,4 +1,4 @@
-"""ctypes binding of lib/libp3d.so (the C ABI declared in include/p3d_render.h and include/p3d_ops.h).
+"""ctypes binding of lib/libp3d.so (the C ABI declared in include/p3d_render.h, include/p3d_ops.h and include/p3d_mesh.h).
 
 The library is loaded lazily on first use and the load FAILS LOUDLY: there is no CPU or
 PyTorch fallback behind any op of this package."""
@@ -67,6 +67,10 @@ _PROTOS = {
     'p3d_copy_async': (C.c_int, [_VP, _VP, C.c_size_t, _VP]),
     'p3d_profile_enable': (None, [C.c_int]),
     'p3d_profile_read': (C.c_int, [C.POINTER(C.c_double), C.POINTER(C.c_uint64), C.c_int, C.c_int]),
+    # include/p3d_mesh.h (marching cubes, panic3d_b200.mesh)
+    'p3d_mc_workspace_bytes': (C.c_size_t, [C.c_int32] * 3),
+    'p3d_mc_count': (C.c_int, [_VP] + [C.c_int32] * 3 + [C.c_double, _VP, C.c_size_t, C.POINTER(C.c_int64), C.POINTER(C.c_float), _VP]),
+    'p3d_mc_emit': (C.c_int, [_VP] + [C.c_int32] * 3 + [C.c_double, _VP, C.c_size_t, _VP] + [C.c_int64] * 4 + [_VP] * 5 + [_VP]),
 }
 
 
