@@ -1,4 +1,5 @@
-"""ctypes binding of lib/libp3d.so (the C ABI declared in include/p3d_render.h, include/p3d_ops.h and include/p3d_mesh.h).
+"""ctypes binding of lib/libp3d.so (the C ABI declared in include/p3d_render.h, include/p3d_ops.h, include/p3d_mesh.h and
+include/p3d_geom.h).
 
 The library is loaded lazily on first use and the load FAILS LOUDLY: there is no CPU or
 PyTorch fallback behind any op of this package."""
@@ -71,6 +72,12 @@ _PROTOS = {
     'p3d_mc_workspace_bytes': (C.c_size_t, [C.c_int32] * 3),
     'p3d_mc_count': (C.c_int, [_VP] + [C.c_int32] * 3 + [C.c_double, _VP, C.c_size_t, C.POINTER(C.c_int64), C.POINTER(C.c_float), _VP]),
     'p3d_mc_emit': (C.c_int, [_VP] + [C.c_int32] * 3 + [C.c_double, _VP, C.c_size_t, _VP] + [C.c_int64] * 4 + [_VP] * 5 + [_VP]),
+    # include/p3d_geom.h (surface sampling, BVH, point-to-mesh distance; panic3d_b200.metrics3d)
+    'p3d_surface_sample_workspace_bytes': (C.c_size_t, [C.c_int64]),
+    'p3d_surface_sample': (C.c_int, [_VP, _VP, C.c_int64, C.c_int64, C.c_uint64, C.c_uint32, _VP, _VP, _VP, C.c_size_t] + [_VP] * 5),
+    'p3d_bvh_workspace_bytes': (C.c_size_t, [C.c_int64]),
+    'p3d_bvh_build': (C.c_int, [_VP, _VP, C.c_int64, _VP, C.c_size_t, _VP]),
+    'p3d_point_mesh_distance': (C.c_int, [_VP, C.c_int64, _VP, _VP, C.c_int64, _VP, C.c_size_t] + [_VP] * 5),
 }
 
 
